@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this framework
     python bench.py --impl reference --gpus N --steps K ...  # reference algorithm on host CPU cores
+    python bench.py ... --dump-outputs DIR                   # also write the last timed step's poses
 
 Metric (BASELINE.json): objects/sec, volumetric pose (32^3).  Workload at every N:
 BASELINE config[1] "singleview_3d inference, 32^3 occupancy 3D-CNN, batch=8 objects" -- one
@@ -536,6 +537,16 @@ def bench_chain(dev, model, runner, rank, world, quick):
 
 
 # ------------------------------------------------------------------ our arm
+def dump_outputs(out_dir, arrays):
+    """Write each array as out_dir/<name>.npy, so that two builds run with the same arguments
+    (hence the same seeded inputs) can be compared output for output."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        a = t.detach().cpu().numpy()
+        assert a.dtype in (np.float32, np.float64), (name, a.dtype)
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def run_ours(args, rank, world, local):
     assert torch.cuda.is_available(), "bench.py (our arm) needs a CUDA device; no CPU fallback"
     import morefusion_b200 as mf
@@ -592,6 +603,9 @@ def run_ours(args, rank, world, local):
     torch.cuda.synchronize()
     barrier(world)
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        # the poses of the last timed step; later passes overwrite runner.out
+        dump_outputs(args.dump_outputs, runner.out)
     step_ms = [a.elapsed_time(b) for a, b in ev]
     total_ms = max_over_ranks(sum(step_ms), world, dev)
     # second pass over the same K steps with the step split into three graphs so that the
@@ -835,7 +849,14 @@ def main():
     ap.add_argument("--quick", action="store_true", help="shorter sub-records (icc / chain)")
     ap.add_argument("--mode", default="infer", choices=["infer", "train"],
                     help="infer: BASELINE config 2 (headline); train: config 3 (data-parallel step)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the poses of the last timed step (rot, trans, conf of rank 0) "
+                         "as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.mode != "infer"):
+        ap.error("--dump-outputs applies to the inference arm (--impl ours --mode infer)")
     if args.impl == "reference":
         # host-CPU arm: rank 0 alone works; other ranks exit 0 without joining any group
         run_reference(args, int(os.environ.get("RANK", "0")), 1)

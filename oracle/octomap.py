@@ -29,9 +29,10 @@ clamped to [0.1192, 0.971]; ``getOccupancy`` is evaluated in double.  An octree 
 observationally a flat key -> log-odds map for ``search`` at depth 0 (a pruned parent carries its
 children's common value and unknown cells stay unknown), which is what this class stores.
 
-The assembly of the three grids from these primitives IS pinned: tests/test_oracle_vs_reference.py
-runs the reference's own ``get_target_grids`` / ``integrate`` code on top of this module
-(oracle/ref_harness/shim.py) and compares with ``get_target_grids`` below.
+The assembly of the three grids from these primitives IS pinned: oracle/ref_harness/gen_golden.py
+runs the reference's own ``get_target_grids`` / ``integrate`` code on top of this module into
+tests/golden/octree_mapping*.npz, which tests/test_oracle_golden.py compares with
+``get_target_grids`` below.
 """
 
 import math

@@ -15,6 +15,8 @@ link, see shim.install) and, for ``octree_mapping``, the OctoMap stand-in
 ``MultiInstanceOctreeMapping`` code runs on the restated ``OcTree``).
 """
 
+import hashlib
+import json
 import os
 import sys
 
@@ -25,13 +27,30 @@ from . import shim
 ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 OUT = os.path.join(ROOT, "tests", "golden")
 F32 = np.float32
+# SHA-256 of every array the generator wrote, so that the committed fixtures can be checked
+# against the reference's output where the reference itself is not available
+DIGESTS = "reference_digests.json"
+_WRITTEN = []
 
 
 def _save(name, **kw):
     os.makedirs(OUT, exist_ok=True)
     path = os.path.join(OUT, name + ".npz")
     np.savez_compressed(path, **kw)
+    _WRITTEN.append(name + ".npz")
     print("wrote", path, os.path.getsize(path), "bytes")
+
+
+def array_digest(a):
+    a = np.ascontiguousarray(a)
+    h = hashlib.sha256(f"{a.dtype.str}{a.shape}".encode())
+    h.update(a.tobytes())
+    return h.hexdigest()
+
+
+def file_digests(path):
+    with np.load(path) as z:
+        return {k: array_digest(z[k]) for k in sorted(z.files)}
 
 
 def _geo(name):
@@ -389,6 +408,7 @@ def gen_octree_mapping_update():
 
 def main():
     assert shim.reference_available(), "needs /root/reference"
+    _WRITTEN.clear()
     gen_octree_mapping()
     gen_octree_mapping_update()
     gen_average_distance()
@@ -398,6 +418,10 @@ def main():
     gen_occupancy()
     gen_transforms()
     gen_icc()
+    digests = {f: file_digests(os.path.join(OUT, f)) for f in sorted(_WRITTEN)}
+    with open(os.path.join(OUT, DIGESTS), "w") as f:
+        json.dump(digests, f, indent=1, sort_keys=True)
+        f.write("\n")
 
 
 if __name__ == "__main__":

@@ -2,7 +2,7 @@
 (check_iterative_collision_check_link.py:44-79: Adam(0.01), translation alpha x0.1, 100
 iterations, sdf_offset=0.02) that the GPU closed-loop parity tests compare with.
 
-TEST INFRASTRUCTURE ONLY.  Run in the dev container (needs /root/reference for `ref3`):
+TEST INFRASTRUCTURE ONLY:
 
     python -m oracle.ref_harness.gen_icc_closed_loop [seed3 seed4 ref3]
 
@@ -10,7 +10,8 @@ TEST INFRASTRUCTURE ONLY.  Run in the dev container (needs /root/reference for `
                   inputs are regenerated from the seed at test time, only the oracle's outputs
                   (q, t, loss history) and a checksum of the inputs are stored.
   ref3            the reference's committed 3-object scene
-                  (/root/reference/examples/ycb_video/pose_refinement/data/0000000{0,1,2}.npz:
+                  (examples/ycb_video/pose_refinement/data/0000000{0,1,2}.npz, stored under
+                  tests/golden/pose_refinement_scene/:
                   transform_init, pitch, origin, grid_target, grid_nontarget_empty copied
                   verbatim).  The fixture lacks the SDF samples (models.get_sdf needs the YCB
                   download, check_iterative_collision_check_link.py:30), so points/sdf are an
@@ -34,7 +35,8 @@ if ROOT not in sys.path:
 from oracle import icc as oicc  # noqa: E402
 
 OUT = os.path.join(ROOT, "tests", "golden")
-REF_DATA = "/root/reference/examples/ycb_video/pose_refinement/data"
+# the reference's examples/ycb_video/pose_refinement/data/0000000{0,1,2}.npz, stored verbatim
+REF_DATA = os.path.join(OUT, "pose_refinement_scene")
 F32 = np.float32
 
 

@@ -16,9 +16,8 @@ from where they lie, under
     i = 0..n-1 (one legal schedule of the GPU execution; for the racy
     index-selection kernels it is the schedule the oracle's tie-break mirrors).
 
-Used by gen_golden.py to produce tests/golden/*.npz and by
-tests/test_oracle_vs_reference.py (skipped when /root/reference is absent,
-as on the GPU box).
+Used by gen_golden.py to produce tests/golden/*.npz and the SHA-256 record
+of them that tests/test_oracle_vs_reference.py checks.
 """
 
 import ctypes
